@@ -2,7 +2,7 @@
 """Benchmark of the ResShift denoising hot path (BASELINE.json metric: 256x256 x4-SR images/sec at 15
 steps; ms/denoise-step).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: the full T=15-step residual-shift sampling loop
 (denoiser forward + p_sample update per step) for a batch of 16 latents of 64x64 (= sixteen 256x256 x4-SR
@@ -321,6 +321,26 @@ def newest_ncu_summary():
     return (tot / n if n else None), tp, f.name
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: Path, arrays: dict):
+    """Writes what the timed path returned in its last step as <out_dir>/<name>.npy (float32), so that two builds run
+    with the same arguments (same seeded inputs) can be compared output for output.  An output larger than
+    DUMP_MAX_BYTES in all keeps a fixed, seeded sample of its images (leading axis)."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    total = sum(a.numel() * 4 for a in arrays.values())
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        if total > DUMP_MAX_BYTES:
+            n = a.shape[0]
+            keep = max(1, int(n * DUMP_MAX_BYTES // total))
+            a = a[np.sort(np.random.default_rng(0).choice(n, keep, replace=False))]
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a, dtype=np.float32))
+    log(f"outputs of the last timed step written to {out_dir}")
+
+
 def run_gpu(args):
     import faulthandler
     faulthandler.dump_traceback_later(900, exit=True)
@@ -407,6 +427,8 @@ def run_gpu(args):
     ms_total = t_ms.item()
     ms_per_step = ms_total / args.steps
     value = world * B / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), {"final_latent": gathered["all"] if world > 1 else out})
 
     if args.quick:       # A/B and ablation runs: only the device-resident figure
         if rank == 0:
@@ -616,7 +638,13 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-bookends", action="store_true")
     ap.add_argument("--quick", action="store_true", help="device-resident timing only (A/B and ablation runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the final latents of the last timed step to DIR/final_latent.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the native path; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -144,77 +144,65 @@ def test_tile_cost_model_invariants_for_the_model_layers():
     assert _tile_config(128, 320, 45)["persist"] == 0
 
 
-def test_tile_starts_match_reference_image_splitter():
+def test_tile_starts_match_reference_image_splitter(golden_dir):
     """The sampler's tiling of large inputs must cut the same tiles as the reference's ImageSpliterTh
-    (utils/util_image.py:889-979).  Compared against the reference class itself when its tree is present (this
-    container), against a table generated from it otherwise (the GPU box)."""
-    import sys
+    (utils/util_image.py:889-979): the row / column starts it computed are stored in tests/golden/image_splitter.json
+    (oracle/make_golden_splitter.py)."""
     from resshift_b200.sampler import tile_starts
     table = {(300, 128, 128): [0, 128, 172], (256, 128, 128): [0, 128], (240, 128, 112): [0, 112], (500, 128, 112): [0, 112, 224, 336, 372],
              (100, 128, 64): [0], (129, 128, 128): [0, 1], (592, 256, 224): [0, 224, 336], (448, 256, 224): [0, 192]}
     for (n, ps, st), want in table.items():
         assert tile_starts(n, ps, st) == want, (n, ps, st)
-    ref_root = Path("/root/reference")
-    if not ref_root.exists():
-        return
-    sys.path[:0] = [str(ROOT / "oracle" / "_shims"), str(ref_root)]
-    try:
-        from utils.util_image import ImageSpliterTh
-        for n in list(range(1, 70)) + [100, 127, 128, 129, 200, 255, 256, 257, 300, 448, 500, 592, 1000]:
-            for ps, st in [(16, 16), (16, 12), (32, 28), (64, 64), (128, 112), (256, 224)]:
-                sp = ImageSpliterTh(torch.zeros(1, 1, n, max(n // 2, 1)), ps, st, sf=1)
-                assert tile_starts(n, ps, st) == sp.height_starts_list, (n, ps, st)
-                assert tile_starts(max(n // 2, 1), ps, st) == sp.width_starts_list, (n, ps, st)
-    finally:
-        del sys.path[:2]
-        for m in [k for k in sys.modules if k == "utils" or k.startswith("utils.")]:
-            del sys.modules[m]
+    cases = json.loads((golden_dir / "image_splitter.json").read_text())["tile_starts"]
+    assert len(cases) == 82 * 6
+    for c in cases:
+        n, ps, st = c["n"], c["patch"], c["stride"]
+        assert tile_starts(n, ps, st) == c["height_starts"], (n, ps, st)
+        assert tile_starts(max(n // 2, 1), ps, st) == c["width_starts"], (n, ps, st)
 
 
-def test_tile_plan_matches_reference_splitter():
+def test_tile_plan_matches_reference_splitter(golden_dir):
     """Host side of the tiled pass: plan_tiles must enumerate exactly the tiles, in exactly the batches, that iterating
     the reference's ImageSpliterTh(extra_bs=chop_bs) yields (utils/util_image.py:889-960) — the per-call batch shape fixes
-    the noise draw, the order fixes the overlap-average's summation order.  (The device side — rs_op_tile_gather against
+    the noise draw, the order fixes the overlap-average's summation order.  The reference's tiles are stored in
+    tests/golden/image_splitter.json (oracle/make_golden_splitter.py).  (The device side — rs_op_tile_gather against
     the reference-form accumulate — is tests/test_gpu_vq.py::test_image_edges_match_torch and the tiled GPU test.)"""
-    import sys
     from resshift_b200.sampler import plan_tiles
-    ref_root = Path("/root/reference")
-    if not ref_root.exists():
-        pytest.skip("reference tree not present")
-    sys.path[:0] = [str(ROOT / "oracle" / "_shims"), str(ref_root)]
-    try:
-        from utils.util_image import ImageSpliterTh
-        for (h, w, ps, st, sf, bs) in [(75, 50, 32, 28, 4, 1), (148, 112, 128, 112, 4, 3), (64, 200, 64, 48, 4, 8),
-                                       (40, 40, 64, 48, 4, 2), (592 // 4, 448 // 4, 128, 112, 4, 4), (512, 700, 256, 224, 1, 5)]:
-            im = torch.zeros(2, 3, h, w)
-            sp = ImageSpliterTh(im, ps, st, sf=sf, extra_bs=bs)
-            ref_groups, ref_shapes = [], []
-            for pch, idx in sp:                           # (index_infos' ends may exceed the image; the slice clips them)
-                ref_groups.append([(i[0] // sf, i[2] // sf) for i in idx])
-                ref_shapes.append((pch.shape[0], pch.shape[2], pch.shape[3]))
-            hs_list, ws_list, th, tw, groups = plan_tiles(h, w, ps, st, bs)
-            if h <= ps and w <= ps:                       # the reference does not tile at all in this case (sampler.py:186)
-                assert groups == [[(0, 0)]]
-                continue
-            assert groups == ref_groups, (h, w, ps, st, bs)
-            assert [(2 * len(g), th, tw) for g in groups] == ref_shapes, (h, w, ps, st, bs)
-            assert hs_list == sp.height_starts_list and ws_list == sp.width_starts_list
-    finally:
-        del sys.path[:2]
-        for m in [k for k in sys.modules if k == "utils" or k.startswith("utils.")]:
-            del sys.modules[m]
+    cases = json.loads((golden_dir / "image_splitter.json").read_text())["plan_tiles"]
+    assert len(cases) == 6
+    for c in cases:
+        h, w, ps, st, bs = c["h"], c["w"], c["patch"], c["stride"], c["bs"]
+        # (the reference's index_infos ends may exceed the image; its slice clips them)
+        ref_groups = [[tuple(s) for s in grp] for grp in c["groups"]]
+        ref_shapes = [tuple(s) for s in c["patch_shapes"]]
+        hs_list, ws_list, th, tw, groups = plan_tiles(h, w, ps, st, bs)
+        if h <= ps and w <= ps:                       # the reference does not tile at all in this case (sampler.py:186)
+            assert groups == [[(0, 0)]]
+            continue
+        assert groups == ref_groups, (h, w, ps, st, bs)
+        assert [(2 * len(g), th, tw) for g in groups] == ref_shapes, (h, w, ps, st, bs)
+        assert hs_list == c["height_starts"] and ws_list == c["width_starts"]
+
+
+def _stand_in_reference_tree(root: Path) -> Path:
+    """A tree with the reference's layout where the overlay must take effect: top-level `sampler`, and a `models`
+    namespace package (no __init__.py) holding `unet`, `script_util` and `basic_ops`.  The stand-ins define none of the
+    names the probe reads, so a stand-in imported in place of the overlay fails the probe."""
+    (root / "models").mkdir(parents=True)
+    for rel in ("sampler.py", "models/unet.py", "models/script_util.py", "models/basic_ops.py"):
+        (root / rel).write_text("FROM_REFERENCE_TREE = True\n")
+    return root
 
 
 def test_overlay_resolves_reference_module_names_to_this_package(tmp_path):
     """`python -m resshift_b200.launch <script>` must make `sampler`, `models.unet`, `models.script_util` resolve to this
     package while every other `models.*` module still comes from the reference tree (namespace package), exactly as an
-    unmodified reference entry script imports them."""
+    unmodified reference entry script imports them.  The reference tree is a stand-in with the same module layout."""
     import subprocess
     import sys
-    ref_root = Path("/root/reference")
-    if not ref_root.exists():
-        pytest.skip("reference tree not present")
-    probe = tmp_path / "probe_entry.py"
+    ref_root = _stand_in_reference_tree(tmp_path / "reference")
+    probe = tmp_path / "entry" / "probe_entry.py"
+    probe.parent.mkdir()
     probe.write_text(
         "import sampler, models.unet, models.script_util\n"
         "import models.basic_ops as ref_ops\n"
