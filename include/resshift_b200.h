@@ -220,6 +220,12 @@ int rs_op_swin_attn(const void* x, int N, int H, int W, int E, int heads, int sh
                     const float* gamma, const float* beta, const void* wqkv_packed, const float* bqkv, const float* relbias_dense,
                     const void* wproj_packed, const float* bproj, void* y, float* part_out, float* gstat_out_or_null,
                     uint32_t* counters_or_null, void* stream);
+/* fused single-head attention of the VQ-GAN bottleneck (reference AttnBlock.forward between the q / k / v convolutions
+ * and proj_out, ldm/modules/diffusionmodules/model.py:180-203): per image n, out[n] = softmax(q[n] k[n]^T C^-1/2) v[n]
+ * + v_bias with q, k [N][T][C] fp16, vt = v^T WITHOUT the bias [N][C][T] fp16, v_bias fp32 [C], out [N][T][C] fp16.
+ * C a multiple of 64 in [64, 512], T a multiple of 64 (any size: the T x T scores never leave the chip). */
+int rs_op_vq_attention(const void* q, const void* k, const void* vt, const float* v_bias, int N, int T, int C, void* out,
+                       void* stream);
 /* fused Swin MLP (reference models/swin_transformer.py:17-33,279): out = residual + fc2(GELU(fc1(x))) */
 int rs_op_mlp(const void* x, int N, int H, int W, int E, int Hd, const void* w1_packed, const float* b1,
               const void* w2_packed, const float* b2, const void* residual, void* out, void* dbg_timeline_or_null,

@@ -92,6 +92,7 @@ _SIGNATURES = {
     "rs_op_window_attention": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "rs_op_swin_attn": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P, _P,
                                   _P, _P, _P, _P, _P]),
+    "rs_op_vq_attention": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "rs_op_mlp": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]),
     "rs_debug_tile_config": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32)]),
     "rs_debug_swin_timeline": (C.c_int, [_P]),

@@ -257,7 +257,7 @@ int build_inventory(rs_engine& e) {
 // ------------------------------------------------------------------------------------------------
 namespace {
 
-enum OpKind { OP_CONV, OP_GN, OP_ATTN, OP_UPSAMPLE, OP_MLP, OP_SOFTMAX, OP_FORK, OP_JOIN, OP_SWIN_ATTN };
+enum OpKind { OP_CONV, OP_GN, OP_ATTN, OP_UPSAMPLE, OP_MLP, OP_SOFTMAX, OP_FORK, OP_JOIN, OP_SWIN_ATTN, OP_VQ_ATTN };
 
 struct Tensor {
   size_t bytes = 0;
@@ -284,6 +284,9 @@ struct Op {
   MlpDesc mlp;
   // fused attention half of a Swin block (norm1 + qkv + window attention + proj + residual)
   SwinAttnDesc swin;
+  // fused single-head attention of the VQ-GAN bottleneck: Q, K [N][T][C], V^T [N][C][T] -> out [N][T][C] (vq.inc)
+  View vqa_q, vqa_k, vqa_vt, vqa_out;
+  VqAttnDesc vqa;
   std::string blk_name;
   std::string w2_name, b2_name;
   std::string w_name, b_name, g_name;   // parameter names resolved at bind
@@ -961,6 +964,16 @@ int bind_ops(rs_plan& P, std::vector<Op>& ops) {
       }
       int rc = swin_attn_finalize(w); if (rc) return rc;
       ++P.launches;
+    } else if (op.kind == OP_VQ_ATTN) {
+      resolve(P, op.vqa_q); resolve(P, op.vqa_k); resolve(P, op.vqa_vt); resolve(P, op.vqa_out);
+      VqAttnDesc& d = op.vqa;
+      d.q = op.vqa_q.ptr; d.k = op.vqa_k.ptr; d.vt = op.vqa_vt.ptr; d.out = op.vqa_out.ptr; d.ld_out = op.vqa_out.ld;
+      d.N = op.vqa_q.N; d.T = op.vqa_q.H * op.vqa_q.W; d.C = op.vqa_q.C;
+      d.bias = E.at<float>(op.b_name);
+      RS_CHECK(d.bias != nullptr, "missing " + op.b_name);
+      RS_CHECK(op.vqa_q.ld == d.C && op.vqa_k.ld == d.C && op.vqa_vt.ld == d.T, "fused VQ attention: dense operands");
+      int rc = vq_attn_finalize(d); if (rc) return rc;
+      ++P.launches;
     } else if (op.kind == OP_FORK || op.kind == OP_JOIN) {
       // stream structure only
     } else if (op.kind == OP_SOFTMAX) {
@@ -987,7 +1000,7 @@ struct Prof {
 };
 
 // RS_SKIP_KINDS (timing ablation only — results are garbage): bit 0 conv3x3, 1 conv1x1 / linear, 2 GroupNorm, 3 window
-// attention, 4 upsample, 5 fused MLP.  The time a kernel family really costs inside the graph-replayed step is the
+// attention (also the fused Swin and VQ-GAN attention kernels), 4 upsample, 5 fused MLP.  The time a kernel family really costs inside the graph-replayed step is the
 // difference between the full step and the step without it (per-launch events and ncu both over-state small kernels).
 inline bool op_skipped(const Op& op) {
   static const int skip = env_int("RS_SKIP_KINDS", 0);
@@ -999,6 +1012,7 @@ inline bool op_skipped(const Op& op) {
     case OP_UPSAMPLE: return (skip >> 4) & 1;
     case OP_MLP: return (skip >> 5) & 1;
     case OP_SWIN_ATTN: return (skip >> 3) & 1;
+    case OP_VQ_ATTN: return (skip >> 3) & 1;
     case OP_SOFTMAX: case OP_FORK: case OP_JOIN: return false;
   }
   return false;
@@ -1037,6 +1051,7 @@ int run_ops(rs_plan& P, const std::vector<Op>& ops, const float* film_base, long
       }
       case OP_MLP: rc = mlp_launch(op.mlp, st); break;
       case OP_SWIN_ATTN: rc = swin_attn_launch(op.swin, st); break;
+      case OP_VQ_ATTN: rc = vq_attn_launch(op.vqa, st); break;
       case OP_ATTN:
         rc = attn_launch(op.a_in, op.a_out, op.a_bias, P.e->cfg.swin_heads, P.e->cfg.swin_embed_dim, op.a_shift, st);
         break;
@@ -1309,6 +1324,9 @@ static void collect_profile(const rs_plan& P, const Prof& prof, double* ms, char
       snprintf(d, desc_stride, "attn %dx%d shift=%d", op.a_in.H, op.a_in.W, op.a_shift);
     } else if (op.kind == OP_SWIN_ATTN) {
       snprintf(d, desc_stride, "swin_attn %dx%d shift=%d grid=%d", op.swin.x.H, op.swin.x.W, op.swin.shift, op.swin.grid);
+    } else if (op.kind == OP_VQ_ATTN) {
+      snprintf(d, desc_stride, "vq_attn %dx%d T=%d C=%d grid=%ux%ux%u", op.vqa_q.H, op.vqa_q.W, op.vqa.T, op.vqa.C, op.vqa.grid.x,
+               op.vqa.grid.y, op.vqa.grid.z);
     } else if (op.kind == OP_FORK || op.kind == OP_JOIN) {
       snprintf(d, desc_stride, "%s", op.kind == OP_FORK ? "fork" : "join");
     } else if (op.kind == OP_SOFTMAX) {

@@ -17,6 +17,7 @@
 #include "window_attn.cuh"
 #include "swin_attn_fused.cuh"
 #include "swin_attn_tc.cuh"
+#include "vq_attn_tc.cuh"
 
 namespace rs {
 
@@ -486,6 +487,7 @@ inline int conv_init() {   // once per process, outside any stream capture
     RS_CUDA_OK(cudaFuncSetAttribute(swin_attn_fused_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SwinSmem<64>::total));
     RS_CUDA_OK(cudaFuncSetAttribute(swin_attn_tc_kernel<192>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SwinTcSmem<192>::total));
     RS_CUDA_OK(cudaFuncSetAttribute(swin_attn_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SwinTcSmem<64>::total));
+    RS_CUDA_OK(cudaFuncSetAttribute(vq_attn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, vqa_smem_bytes(512)));
     attr_set = true;
   }
   return 0;
@@ -764,6 +766,57 @@ inline int swin_attn_launch(const SwinAttnDesc& d, cudaStream_t st) {
   }
   if (d.x.C == 192) (void)launch_k(swin_attn_fused_kernel<192>, dim3(d.grid), dim3(kSwinThreads), SwinSmem<192>::total, st, d.prm);
   else (void)launch_k(swin_attn_fused_kernel<64>, dim3(d.grid), dim3(kSwinThreads), SwinSmem<64>::total, st, d.prm);
+  RS_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+// Fused single-head attention of the VQ-GAN bottleneck (vq_attn_tc.cuh): q, k [N][T][C], vt [N][C][T] fp16, out
+// [N][T][ld_out] fp16.
+struct VqAttnDesc {
+  const __half* q = nullptr; const __half* k = nullptr; const __half* vt = nullptr;
+  const float* bias = nullptr;
+  __half* out = nullptr; int ld_out = 0;
+  int N = 0, T = 0, C = 0;
+  VqAttnParams prm;
+  dim3 grid;
+};
+inline bool vq_attn_supported(int T, int C) { return C % 64 == 0 && C >= 64 && C <= 512 && T % 64 == 0 && T >= 64; }
+// 3-D fp16 map {d0, d1, d2} (d0 contiguous), 128B swizzle, box {64, box1, 1}
+inline int encode_3d_map(CUtensorMap* m, const __half* base, long long d0, long long d1, long long d2, long long s1,
+                         long long s2, int box1) {
+  PFN_encodeTiled enc = get_encode_tiled();
+  RS_CHECK(enc != nullptr, "cuTensorMapEncodeTiled entry point not available (no CUDA driver?)");
+  RS_CHECK((reinterpret_cast<uintptr_t>(base) & 15) == 0 && s1 % 8 == 0 && s2 % 8 == 0, "attention operands: 16-byte rows");
+  cuuint64_t dims[3] = {(cuuint64_t)d0, (cuuint64_t)d1, (cuuint64_t)d2};
+  cuuint64_t strides[2] = {(cuuint64_t)s1 * 2, (cuuint64_t)s2 * 2};
+  cuuint32_t box[3] = {64, (cuuint32_t)box1, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<__half*>(base), dims, strides, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  RS_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled(attention operand) failed with CUresult " + std::to_string((int)r));
+  return 0;
+}
+inline int vq_attn_finalize(VqAttnDesc& d) {
+  RS_CHECK(d.q && d.k && d.vt && d.bias && d.out && d.N > 0, "fused VQ attention: null operand");
+  RS_CHECK(vq_attn_supported(d.T, d.C), "fused VQ attention: C a multiple of 64 in [64, 512], T a multiple of 64");
+  RS_CHECK(d.ld_out >= d.C && d.ld_out % 8 == 0, "fused VQ attention: output row stride");
+  VqAttnParams& p = d.prm;
+  std::memset(&p, 0, sizeof(p));
+  p.T = d.T; p.C = d.C;
+  p.DV = d.C <= 256 ? d.C : d.C / 2;
+  p.n_vc = p.DV > 128 ? 2 : 1;
+  p.VC = p.DV / p.n_vc;
+  p.scale_log2 = 1.4426950408889634f / std::sqrt((float)d.C);
+  p.bias = d.bias; p.out = d.out; p.ld_out = d.ld_out;
+  int rc = encode_3d_map(&p.tmQ, d.q, d.C, d.T, d.N, d.C, (long long)d.T * d.C, 128); if (rc) return rc;
+  rc = encode_3d_map(&p.tmK, d.k, d.C, d.T, d.N, d.C, (long long)d.T * d.C, 128); if (rc) return rc;
+  rc = encode_3d_map(&p.tmVt, d.vt, d.T, d.C, d.N, d.T, (long long)d.T * d.C, p.VC); if (rc) return rc;
+  d.grid = dim3((unsigned)((d.T + 127) / 128), (unsigned)(d.C / p.DV), (unsigned)d.N);
+  return 0;
+}
+inline int vq_attn_launch(const VqAttnDesc& d, cudaStream_t st) {
+  (void)launch_k(vq_attn_tc_kernel, d.grid, dim3(kVqaThreads), (size_t)vqa_smem_bytes(d.C), st, d.prm);
   RS_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -10,7 +10,8 @@ owns every allocation; there is no eager / CPU fallback.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional, Tuple
+from collections import OrderedDict
+from typing import Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -48,7 +49,9 @@ class VQModelTorch(nn.Module):
         self._engine = None
         self._arena: Optional[torch.Tensor] = None
         self._packed_versions: Optional[Tuple] = None
-        self._plans: Dict[Tuple[int, int, int, int], "_VQPlan"] = {}
+        # (direction, batch, H, W) -> plan, least recently used first; at most MAX_PLANS_PER_DIRECTION per direction (a
+        # plan owns its workspace: gigabytes at 2048x2048, and folder inference meets one padded size per image)
+        self._plans: "OrderedDict[Tuple[int, int, int, int], _VQPlan]" = OrderedDict()
         self.last_indices: Optional[torch.Tensor] = None
 
     # ------------------------------------------------------------------ native plumbing
@@ -76,7 +79,7 @@ class VQModelTorch(nn.Module):
             self._arena_ptr = (self._arena.data_ptr() + 255) // 256 * 256
             _lib.check(_lib.lib.rs_unet_set_arena(self._engine, self._arena_ptr))
             self._packed_versions = None
-            self._plans.clear()
+            self._drop_plans()
         return self._engine
 
     def pack_weights(self, force: bool = False):
@@ -97,14 +100,26 @@ class VQModelTorch(nn.Module):
         torch.cuda.current_stream().synchronize()
         self._packed_versions = versions
 
+    MAX_PLANS_PER_DIRECTION = 2
+
+    def _drop_plans(self):
+        for p in self._plans.values():
+            p.close()
+        self._plans.clear()
+
     def plan(self, which: int, batch: int, image_h: int, image_w: int) -> "_VQPlan":
         device = next(self.parameters()).device
         self._ensure_engine(device)
         self.pack_weights()
         key = (which, batch, image_h, image_w)
-        if key not in self._plans:
-            self._plans[key] = _VQPlan(self, which, batch, image_h, image_w, device)
-        return self._plans[key]
+        plan = self._plans.pop(key, None)
+        if plan is None:
+            same = [k for k in self._plans if k[0] == which]
+            while len(same) >= self.MAX_PLANS_PER_DIRECTION:
+                self._plans.pop(same.pop(0)).close()
+            plan = _VQPlan(self._engine, which, batch, image_h, image_w, device)
+        self._plans[key] = plan
+        return plan
 
     # ------------------------------------------------------------------ reference call surface
     @torch.no_grad()
@@ -146,7 +161,7 @@ class VQModelTorch(nn.Module):
 
     def __del__(self):
         try:
-            self._plans.clear()
+            self._drop_plans()
             if self._engine is not None:
                 _lib.lib.rs_unet_destroy(self._engine)
         except Exception:
@@ -154,12 +169,12 @@ class VQModelTorch(nn.Module):
 
 
 class _VQPlan:
-    """VQ-GAN engine bound to (encode | decode, batch, image H, image W): owns the workspace and the native plan."""
+    """VQ-GAN engine bound to (encode | decode, batch, image H, image W): owns the workspace and the native plan.  It keeps
+    no reference to its model (the model's plan cache holds the plans; ``close`` runs before the engine is destroyed)."""
 
-    def __init__(self, model: VQModelTorch, which: int, batch: int, image_h: int, image_w: int, device):
-        self.model = model
+    def __init__(self, engine, which: int, batch: int, image_h: int, image_w: int, device):
         h = C.c_void_p()
-        _lib.check(_lib.lib.rs_vq_plan_create(model._engine, batch, image_h, image_w, which, C.byref(h)))
+        _lib.check(_lib.lib.rs_vq_plan_create(engine, batch, image_h, image_w, which, C.byref(h)))
         self.handle = h
         nbytes = _lib.lib.rs_plan_workspace_bytes(h)
         self.workspace = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
@@ -167,8 +182,16 @@ class _VQPlan:
         _lib.check(_lib.lib.rs_plan_bind(h, self.workspace_ptr))
         self.launches = _lib.lib.rs_plan_num_launches(h)
 
+    def close(self):
+        """Destroy the native plan and release the workspace (work already queued on the stream keeps it alive in torch's
+        stream-ordered allocator)."""
+        if self.handle is not None:
+            _lib.lib.rs_plan_destroy(self.handle)
+            self.handle = None
+            self.workspace = None
+
     def __del__(self):
         try:
-            _lib.lib.rs_plan_destroy(self.handle)
+            self.close()
         except Exception:
             pass
